@@ -365,8 +365,8 @@ def gated_crf_loss(y, image, radius=5, sigma_xy=6.0, sigma_rgb=0.1, weight=1.0):
     contributing nothing to the pairwise product (SURVEY F10)."""
     N, C, H, W = y.shape
     dt = y.dtype
-    xs = torch.arange(W, dtype=dt).view(1, 1, 1, W).expand(N, 1, H, W) / sigma_xy      # :174-181, :154
-    ys = torch.arange(H, dtype=dt).view(1, 1, H, 1).expand(N, 1, H, W) / sigma_xy
+    xs = torch.arange(W, dtype=dt, device=y.device).view(1, 1, 1, W).expand(N, 1, H, W) / sigma_xy      # :174-181, :154
+    ys = torch.arange(H, dtype=dt, device=y.device).view(1, 1, H, 1).expand(N, 1, H, W) / sigma_xy
     inten = F.adaptive_avg_pool2d(image.to(dt), (H, W)) / sigma_rgb                      # :127-132
     feat = torch.cat([xs, ys, inten], 1)
     r = radius

@@ -468,6 +468,9 @@ __global__ void __launch_bounds__(TPB) pdice_bwd_kernel(
 //   mn = minpool3(p), contour = relu(maxpool3(mn) - mn), loss = mean(contour); pools see only in-bounds
 //   pixels (max_pool2d pads with -inf).  Backward routes like autograd: +g to the argmin of the window
 //   that attains the max, -g to the argmin of the centre window (first extremum in row-major scan order).
+//   The atomics add +-1 (integer counts, exact in fp32 in any order) and tv_scale_kernel multiplies by g
+//   afterwards: adding +-g directly rounds partial sums such as 3g, so the result would depend on the
+//   order of the atomics, run to run, and contributions that cancel could leave a residue instead of 0.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float minpool_at(const float* P, int H, int W, int y, int x, int* arg) {
   float best = INFINITY;
@@ -484,7 +487,7 @@ __device__ __forceinline__ float minpool_at(const float* P, int H, int W, int y,
 }
 
 __global__ void __launch_bounds__(TPB) tv_kernel(
-    const float* __restrict__ probs, int planes, int H, int W, float gscale /*go/numel*/, float* __restrict__ gprobs,
+    const float* __restrict__ probs, int planes, int H, int W, float* __restrict__ gcount,
     float* partials, unsigned* ticket, float* out) {
   const long long HW = (long long)H * W, total = (long long)planes * HW;
   float acc[1] = {0.f};
@@ -507,9 +510,9 @@ __global__ void __launch_bounds__(TPB) tv_kernel(
     const float c = mx - mc;
     if (c > 0.f) {
       acc[0] += c;
-      if (gprobs) {
-        atomicAdd(gprobs + pl * HW + argm, gscale);
-        atomicAdd(gprobs + pl * HW + argc, -gscale);
+      if (gcount) {
+        atomicAdd(gcount + pl * HW + argm, 1.f);
+        atomicAdd(gcount + pl * HW + argc, -1.f);
       }
     }
   }
@@ -517,6 +520,10 @@ __global__ void __launch_bounds__(TPB) tv_kernel(
   if (block_reduce_final<1, TPB>(acc, partials, ticket, res)) {
     if (threadIdx.x == 0) out[0] = (float)(res[0] / (double)total);
   }
+}
+
+__global__ void __launch_bounds__(TPB) tv_scale_kernel(float* __restrict__ g, long long total, float gscale /*go/numel*/) {
+  for (long long i = blockIdx.x * (long long)TPB + threadIdx.x; i < total; i += (long long)gridDim.x * TPB) g[i] *= gscale;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -708,7 +715,7 @@ __global__ void __launch_bounds__(TPB) entropy_bwd_kernel(const float* __restric
 //   v = img * p_c;  intra = mean_{n,c} std_{hw}(v)  (unbiased);  inter = mean_n std_c(mean_{hw}(v))  (unbiased over C)
 //   loss = inter - intra.   fwd: per-(n,c) sums S1 = sum v, S2 = sum v^2 (grid = (chunks, N)), finalised by the last
 //   block into stats[n][c] = {mean, std} + stats_n[n] = {mean over classes, std over classes}; bwd is elementwise.
-// A zero standard deviation yields a zero gradient here (the reference's autograd would produce inf/NaN).
+// A zero standard deviation yields a zero gradient, as torch's std backward does (it masks result == 0).
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(TPB) variance_fwd_kernel(const float* __restrict__ image, const float* __restrict__ probs, int N,
                                                            long long HW, float* partials, unsigned* ticket, float* out /*[3]*/,
@@ -991,8 +998,10 @@ WSL_API int wsl_pdice_bwd(const float* probs, const uint8_t* target, const float
 WSL_API int wsl_tv_loss(const float* probs, int planes, int H, int W, float grad_scale, float* gprobs_zeroed, float* out1,
                         float* ws, cudaStream_t stream) {
   const long long total = (long long)planes * H * W;
-  tv_kernel<<<grid_for(total, TPB), TPB, 0, stream>>>(probs, planes, H, W, grad_scale / (float)total, gprobs_zeroed,
-                                                      ws + 64, reinterpret_cast<unsigned*>(ws), out1);
+  tv_kernel<<<grid_for(total, TPB), TPB, 0, stream>>>(probs, planes, H, W, gprobs_zeroed, ws + 64, reinterpret_cast<unsigned*>(ws),
+                                                      out1);
+  if (gprobs_zeroed != nullptr)
+    tv_scale_kernel<<<grid_for(total, TPB * 4), TPB, 0, stream>>>(gprobs_zeroed, total, grad_scale / (float)total);
   return wsl_check_launch("tv_loss");
 }
 
